@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark: batched 1-D FFTs/s at N=1024 complex fp32 (BASELINE.json).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One step = one pass of the hot path over one synthetic batch: `batch` forward transforms followed by
@@ -46,7 +46,25 @@ def parse():
     ap.add_argument("--e2e-batch", type=int, default=1 << 17, help="transforms per e2e step (host buffers)")
     ap.add_argument("--cpu-seconds", type=float, default=12.0, help="target wall time of the cpu_baseline leg")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed step's outputs (a fixed sample of rows) to DIR/forward.npy, DIR/backward.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+DUMP_ROWS = 2048                       # 2 x 2048 transforms x 8 KiB = 32 MiB of outputs
+
+
+def dump_outputs(d, y, z):
+    """forward (y) and backward (z) outputs of the same seeded sample of rows, float32, one (rows, 2N) array each"""
+    import torch
+    os.makedirs(d, exist_ok=True)
+    rows = np.sort(np.random.default_rng(0).choice(y.shape[0], min(y.shape[0], DUMP_ROWS), replace=False))
+    idx = torch.from_numpy(rows).to(y.device)
+    for name, t in (("forward", y), ("backward", z)):
+        np.save(os.path.join(d, name + ".npy"), t.index_select(0, idx).cpu().numpy())
 
 
 # ------------------------------------------------------------------------------------------------ clocks
@@ -308,6 +326,8 @@ def main():
     wall1 = time.time()
     launches = pf.launch_count() - launches0
     clocks = sampler.stop(wall0, wall1) if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, y, z)
     ms = ev0.elapsed_time(ev1)
     fwd_ms = float(np.mean([a.elapsed_time(b) for a, b in fwd_ev]))
     if world > 1:

@@ -41,7 +41,8 @@ def test_device_resident_shards_and_bit_identical_gpus(pf, ref, R):
     m = pf.Multi(N, pf.PFFFT_REAL, 0)
     G = m.ngpus
     xs, ys, nb = [], [], []
-    base = torch.rand((64, N), device="cuda:0") * 2 - 1
+    gen = torch.Generator(device="cuda:0"); gen.manual_seed(N)
+    base = torch.rand((64, N), generator=gen, device="cuda:0") * 2 - 1
     for g in range(G):
         xs.append(base.to("cuda:%d" % g))
         ys.append(torch.empty_like(xs[-1]))

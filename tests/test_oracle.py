@@ -95,9 +95,11 @@ def test_checkers_against_golden_and_numpy(orc, ref, R):
         N = int(key[1:].split("_")[0]); tr = 0 if "_r_" in key else 1
         dtype = np.dtype(np.float32 if key.endswith("f4") else np.float64)
         x = g[key + "_x"]
-        # the golden file IS the reference's output: must reproduce bit-exactly here
-        assert np.array_equal(ref.transform(N, tr, x, 0, True, dtype), g[key + "_fwd_ordered"]), key
-        assert np.array_equal(ref.transform(N, tr, x, 0, False, dtype), g[key + "_fwd_z"]), key
+        fo, fz = ref.transform(N, tr, x, 0, True, dtype), ref.transform(N, tr, x, 0, False, dtype)
+        if R.have_ref():
+            # the golden file IS the reference's output: the reference built into oracle/_ref reproduces it bit-exactly
+            assert np.array_equal(fo, g[key + "_fwd_ordered"]), key
+            assert np.array_equal(fz, g[key + "_fwd_z"]), key
         tol = (2e-6 if dtype == np.float32 else (1e-13 if (N & (N - 1)) == 0 else 2e-7))
         assert R.relmax(orc.transform(N, tr, x, 0, True, dtype), g[key + "_fwd_ordered"]) <= tol, key
         # second opinion: numpy float64 (SURVEY App. D: 1.3e-7 .. 2.8e-7 for float)

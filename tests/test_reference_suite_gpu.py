@@ -32,6 +32,7 @@ CASES = [
 def test_reference_program_passes_against_drop_in_library(exe, args, timeout):
     path = os.path.join(ACC, exe)
     if not os.path.exists(path):
-        pytest.skip("oracle/_ref/acceptance/%s not built (make -C oracle acceptance, needs /root/reference)" % exe)
+        pytest.skip("oracle/_ref/acceptance/%s not built: `make -C oracle acceptance REF=<pffft source tree>` builds the "
+                    "reference's own test programs, which are not part of this repository" % exe)
     r = subprocess.run([path] + args, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True, timeout=timeout)
     assert r.returncode == 0, "%s %s failed (rc=%d):\n%s" % (exe, " ".join(args), r.returncode, r.stdout[-3000:])

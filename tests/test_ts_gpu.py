@@ -88,8 +88,9 @@ def test_two_streams_share_one_plan(pf, ref, R, ts_on):
     """the rings and counters of a plan serve one launch at a time: calls from two streams are ordered by the plan's event"""
     import torch
     N = 32768
-    x1 = torch.rand((64, 2 * N), device="cuda") * 2 - 1
-    x2 = torch.rand((64, 2 * N), device="cuda") * 2 - 1
+    g = torch.Generator(device="cuda"); g.manual_seed(N)
+    x1 = torch.rand((64, 2 * N), generator=g, device="cuda") * 2 - 1
+    x2 = torch.rand((64, 2 * N), generator=g, device="cuda") * 2 - 1
     y1 = torch.empty_like(x1); y2 = torch.empty_like(x2)
     s1, s2 = torch.cuda.Stream(), torch.cuda.Stream()
     torch.cuda.synchronize()
